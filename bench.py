@@ -2,6 +2,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our arm (CUDA)
   python bench.py --impl reference --gpus N --steps K ...   # reference arm (CPU)
+  python bench.py ... --dump-outputs DIR                    # + the last timed step's outputs as .npy
 
 Workload ("config.workload"): batched teacher-student sparse GLM, BASELINE.json
 configs[2]: GaussBernoulliPrior(N=4096, rho=0.1) @ LinearChannel(Gaussian W,
@@ -70,7 +71,17 @@ def parse():
                     help="of those, how many are checked against the CPU oracle (rank 0)")
     ap.add_argument("--no-multi-gpu-blocks", action="store_true",
                     help="N > 1: skip the row_sharded / shared_w blocks")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed for rank 0's instances as DIR/<name>.npy "
+                         "(float64, instances on axis 0): posterior means x_r [B, N], z_r [B, M], variances "
+                         "x_v, z_v [B], records mse / vx / vz _per_iter [B, iters]; a fixed seeded sample of "
+                         "the instances if the whole set exceeds 64 MB")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA arm (--impl ours)")
+    return args
 
 
 # --------------------------------------------------------------------------- clocks
@@ -267,6 +278,22 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT_BYTES = 60 * 10**6      # data of --dump-outputs: with the .npy headers, under 64 MB
+
+
+def dump_outputs(np, out_dir, arrays):
+    """Write {name: array with instances on axis 0} as out_dir/<name>.npy in float64; when the set
+    exceeds DUMP_LIMIT_BYTES, keep the same seeded sample of instances in every array."""
+    B = len(next(iter(arrays.values())))
+    total = sum(np.asarray(a, dtype=np.float64).nbytes for a in arrays.values())
+    keep = np.arange(B)
+    if total > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.RandomState(0).choice(B, max(1, B * DUMP_LIMIT_BYTES // total), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(np.asarray(a)[keep], dtype=np.float64))
+
+
 def gemv_bytes_for_schedule(schedule, R, N, M):
     return {0: 16 * R * (N + M), 1: 8 * R * (2 * N + M), 2: 16 * R * N}[schedule]
 
@@ -371,6 +398,12 @@ def run_ours(args):
     flags = st["flags"].cpu().numpy()
     assert not (flags & 3).any(), "NaN in EP messages during the benchmark"
     mse_final = float(rec["mse"][iters - 1].mean().item())
+    if args.dump_outputs and rank == 0:
+        # before the shortcut schedules below reuse the state
+        got = ep.get_variables_data()
+        dump_outputs(np, args.dump_outputs, {
+            "x_r": got["x"]["r"], "x_v": got["x"]["v"], "z_r": got["z"]["r"], "z_v": got["z"]["v"],
+            **{k + "_per_iter": rec[k].T.cpu().numpy() for k in ("mse", "vx", "vz")}})
 
     # ---- exact shortcut schedules for the Gaussian likelihood, reported separately
     # (SURVEY 8d honesty rule: bytes of the passes each schedule really streams)

@@ -53,3 +53,31 @@ def test_our_arm_has_no_cpu_fallback():
     out = _bench("--steps", "1", "--warmup", "0", "--instances", "1", "--n", "64", "--iters", "2")
     assert out.returncode != 0
     assert not any(ln.startswith("{") for ln in out.stdout.splitlines())
+
+
+def test_arguments_that_would_not_time_or_dump_what_they_say_are_rejected(tmp_path):
+    out = _bench("--impl", "reference", "--steps", "0")
+    assert out.returncode == 2 and "--steps" in out.stderr
+    out = _bench("--impl", "reference", "--dump-outputs", str(tmp_path / "out"))
+    assert out.returncode == 2 and "--dump-outputs" in out.stderr
+    assert not (tmp_path / "out").exists()
+
+
+def test_dump_outputs_writes_float64_and_a_fixed_sample_over_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    import bench
+    rng = np.random.RandomState(1)
+    arrays = {"x_r": rng.rand(40, 30), "x_v": rng.rand(40), "mse_per_iter": rng.rand(40, 5).astype(np.float32)}
+    bench.dump_outputs(np, str(tmp_path / "all"), arrays)
+    for name, a in arrays.items():
+        got = np.load(tmp_path / "all" / (name + ".npy"))
+        assert got.dtype == np.float64 and np.array_equal(got, a)
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 10 * 36 * 8)         # 10 of the 40 instances (36 values each)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(np, str(tmp_path / d), arrays)
+    x_r = np.load(tmp_path / "s1" / "x_r.npy")
+    keep = [int(np.flatnonzero((arrays["x_r"] == row).all(axis=1))[0]) for row in x_r]
+    assert len(keep) == 10 and keep == sorted(keep)
+    for name, a in arrays.items():
+        s1, s2 = np.load(tmp_path / "s1" / (name + ".npy")), np.load(tmp_path / "s2" / (name + ".npy"))
+        assert np.array_equal(s1, np.asarray(a, dtype=np.float64)[keep]) and np.array_equal(s1, s2)

@@ -9,12 +9,13 @@ import pytest
 from numpy.testing import assert_allclose
 
 from tests._emulated_device import emulated_device  # noqa: F401  (fixture)
+from tests.golden import load_sweeps
 from tests.test_gpu_api import _build, _configs, _SeqInit
 
 
 @pytest.fixture(scope="module")
 def sw(golden_dir):
-    return np.load(os.path.join(golden_dir, "sweeps.npz"))
+    return load_sweeps(golden_dir)
 
 
 @pytest.mark.parametrize("idx", [0, 1, 2, 6, 8])

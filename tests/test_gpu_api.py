@@ -7,6 +7,8 @@ import numpy as np
 import pytest
 from numpy.testing import assert_allclose
 
+from tests.golden import load_sweeps
+
 pytestmark = pytest.mark.gpu
 
 
@@ -19,7 +21,7 @@ def _need_cuda():
 
 @pytest.fixture(scope="module")
 def sw(golden_dir):
-    return np.load(os.path.join(golden_dir, "sweeps.npz"))
+    return load_sweeps(golden_dir)
 
 
 def _configs(sw):

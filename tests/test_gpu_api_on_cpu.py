@@ -19,11 +19,12 @@ import pytest
 
 from tests._emulated_device import emulated_device  # noqa: F401  (fixture)
 from tests import test_gpu_api as G
+from tests.golden import load_sweeps
 
 
 @pytest.fixture(scope="module")
 def sw(golden_dir):
-    return np.load(os.path.join(golden_dir, "sweeps.npz"))
+    return load_sweeps(golden_dir)
 
 
 @pytest.fixture(scope="module")

@@ -42,8 +42,9 @@ def _sum_over_ranks(dist, v):
     return out
 
 
-def _worker(rank, world, port, golden, name, out_path, backend):
+def _worker(rank, world, port, golden_dir, name, out_path, backend):
     import torch
+    from tests.golden import load_sweeps
     dist = _init(rank, world, port)
     from tramp_b200 import ops
     from tramp_b200.priors import get_prior
@@ -52,7 +53,7 @@ def _worker(rank, world, port, golden, name, out_path, backend):
     from tramp_b200.variables import SISOVariable as V
     from tramp_b200.algos import ExpectationPropagation, TrackErrors
     from tramp_b200.distributed import instance_shard
-    sw = np.load(golden)
+    sw = load_sweeps(golden_dir)
     cfg = [c for c in json.loads(str(sw["configs"])) if c["name"] == name][0]
     W = sw[name + "_W"]
     M, N = W.shape
@@ -89,14 +90,14 @@ def test_row_sharded_instance_matches_reference(golden_dir, tmp_path, name, back
     library baseline (local GEMVs + NCCL all-reduce, staged from Python)."""
     import torch
     import torch.multiprocessing as mp
+    from tests.golden import load_sweeps
     if not torch.cuda.is_available():
         pytest.skip("no CUDA device")
     world = 2
-    golden = os.path.join(golden_dir, "sweeps.npz")
     out = str(tmp_path / "rank%d.npz")
-    mp.spawn(_worker, args=(world, 29600 + os.getpid() % 300, golden, name, out, backend), nprocs=world,
+    mp.spawn(_worker, args=(world, 29600 + os.getpid() % 300, golden_dir, name, out, backend), nprocs=world,
              join=True)
-    sw = np.load(golden)
+    sw = load_sweeps(golden_dir)
     res = [np.load(out % r) for r in range(world)]
     for r in res:
         np.testing.assert_allclose(r["mse"], sw[name + "_mse"], rtol=1e-9)

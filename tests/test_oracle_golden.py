@@ -7,6 +7,7 @@ import pytest
 from numpy.testing import assert_allclose
 
 from oracle import tramp_oracle as orc
+from tests.golden import load_sweeps
 from tests.golden.make_golden_specs import PRIOR_SPECS, LIK_SPECS, TRUNC_CASES
 
 RTOL = 1e-12
@@ -24,7 +25,7 @@ def lin(golden_dir):
 
 @pytest.fixture(scope="module")
 def sw(golden_dir):
-    return np.load(os.path.join(golden_dir, "sweeps.npz"))
+    return load_sweeps(golden_dir)
 
 
 @pytest.mark.parametrize("i", range(len(PRIOR_SPECS)))
@@ -112,7 +113,7 @@ def _configs(sw):
 
 
 def _init_from(sw, name):
-    if f"{name}_init_e1_a" not in sw.files:
+    if f"{name}_init_e1_a" not in sw:
         return None
     return {f"e{k}": (float(sw[f"{name}_init_e{k}_a"]), sw[f"{name}_init_e{k}_b"])
             for k in range(1, 9)}

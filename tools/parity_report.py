@@ -6,8 +6,9 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from tests.test_gpu_api import _build, _SeqInit, _configs
 from tramp_b200.algos import ExpectationPropagation, TrackErrors, TrackEvolution, JoinCallback
+from tests.golden import load_sweeps
 
-sw = np.load("tests/golden/sweeps.npz")
+sw = load_sweeps("tests/golden")
 report = {}
 for cfg in _configs(sw):
     name = cfg["name"]
