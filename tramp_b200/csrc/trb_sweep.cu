@@ -413,6 +413,8 @@ extern "C" void trb_set_update_kernels(int mask) {
 static int check_sweep(const trb_sweep* sw) {
   TRB_CHECK_ARG(sw, "null sweep descriptor");
   TRB_CHECK_ARG(sw->B > 0 && sw->N > 0 && sw->M > 0 && sw->R > 0, "bad shape");
+  // every per-instance launch of the sweep puts the instance index in gridDim.y
+  TRB_CHECK_ARG(sw->B <= 65535, "B > 65535");
   TRB_CHECK_ARG(sw->R <= sw->N && sw->R <= sw->M, "R must be <= min(N, M)");
   TRB_CHECK_ARG(sw->y, "null observation");
   TRB_CHECK_ARG(sw->edge_a && sw->b1 && sw->b3 && sw->b5 && sw->b7, "null message buffer");
